@@ -3,6 +3,7 @@
 
     python bench.py --gpus 1 --steps K --warmup W            # our sm_100a backend
     python bench.py --impl reference --gpus 1 --steps K ...  # the reference's own CUDA kernels (oracle/_ref)
+    python bench.py ... --dump-outputs DIR                   # + what the last timed step computed, as DIR/<name>.npy
 
 A "step" is ONE outer iteration of DirectBA::BundleAdjustment (surfel activation + geometry optimisation +
 pose optimisation of every keyframe, direct_ba_alternating.cc:345-717) on a seeded synthetic 640x480 scene,
@@ -32,6 +33,10 @@ os.environ.setdefault("OMP_PLACES", "cores")
 
 METRIC = "surfel_keyframe_residuals_per_second_per_BA_iteration"
 UNIT = "residuals/s"
+# --dump-outputs: at most this many surfels (a fixed, seeded sample of a larger map) -> 8 rows + flags + indices, 44 MB
+DUMP_SURFELS = 1 << 20
+DUMP_RESULT_FIELDS = ("iterations_done", "converged", "depth_residual_count", "descriptor_residual_count", "cost",
+                      "pose_iterations_total", "surfels_deleted", "surfels_size", "surfels_created", "surfels_merged")
 
 
 def load_peaks():
@@ -277,6 +282,9 @@ def run_ours(args, scene, rank, world):
                 "kernel_share_of_step": prof["pose_ms"] / ms_total,
                 "pairs_per_s": prof["n_pair"] / pose_s if pose_s > 0 else 0.0}
 
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ba, res)
+
     multi_gpu_check = None
     if world > 1:
         multi_gpu_check = check_replicas(scene, ba, step, dev, rank, world)
@@ -335,6 +343,23 @@ def run_ours(args, scene, rank, world):
                                         "balanced by measured work (1 all-reduce of K x 17 floats); NCCL over NVLink")
         dist.barrier(device_ids=[dev.index])
     return out
+
+
+def dump_outputs(out_dir, ba, res):
+    """What the last timed step handed back to a caller, as float32 / float64 arrays in out_dir: keyframe poses and
+    activations, the BundleAdjustment result counters (DUMP_RESULT_FIELDS) and the surfel rows 0-7 (bit patterns of the packed
+    rows kept) with the active flags, of every surfel or of a fixed, seeded sample of DUMP_SURFELS of them."""
+    os.makedirs(out_dir, exist_ok=True)
+    poses, act = ba.GetKeyframeStates()
+    rows, flags = ba.GetSurfelsHost(), ba.GetActiveHost()
+    n = rows.shape[1]
+    cols = np.arange(n) if n <= DUMP_SURFELS else np.sort(np.random.default_rng(0).choice(n, DUMP_SURFELS, replace=False))
+    out = {"keyframe_poses": poses.astype(np.float32), "keyframe_activations": act.astype(np.float64),
+           "ba_result": np.array([getattr(res, f) for f in DUMP_RESULT_FIELDS], np.float64),
+           "surfel_rows": np.ascontiguousarray(rows[:8, cols], np.float32), "surfel_active": flags[cols].astype(np.float32),
+           "surfel_index": cols.astype(np.float64)}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def check_replicas(scene, ba, step, dev, rank, world):
@@ -597,7 +622,10 @@ def _main(saved_stdout):
     ap.add_argument("--intrinsics", action="store_true",
                     help="optimise depth intrinsics + depth deformation and colour intrinsics inside the step (the cfg4 configuration)")
     ap.add_argument("--residuals-override", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))

@@ -2,16 +2,25 @@
 compiled by oracle/build_ref.sh) behind oracle/ref_driver.cu.
 
 TEST / BASELINE INFRASTRUCTURE ONLY.  Needs a GPU; `available()` tells whether it can be used.
+
+The GPU tests do not need the library: `reference(scene, ...)` replays what RefDirectBA returned, call by call, when the
+test ran against the reference's kernels with BADBA_RECORD_REFERENCE=<dir> set (tests/golden/reference/, one file per
+test).  A large output is recorded in part (`Sample`), with the digest of the whole array.
 """
 from __future__ import annotations
 
+import base64
 import ctypes as C
+import hashlib
+import json
 import os
+import re
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_ref", "libbadslam_ref.so")
+RECORDED = os.path.join(os.path.dirname(_HERE), "tests", "golden", "reference")
 
 
 class Config(C.Structure):
@@ -365,3 +374,180 @@ class RefDirectBA:
 
     def launch_count(self):
         return int(self.l.ref_launch_count(self.h))
+
+
+# ---- recorded runs of RefDirectBA ---------------------------------------------------------------------------------------
+
+WHOLE = 256      # arrays up to this many elements are recorded whole
+# outputs (method: tuple positions) that the tests only compare bit for bit (`identical`): recorded as their digest alone
+DIGEST_ONLY = {"odometry_level": (0, 2), "preprocess_frame": (3,)}
+
+
+class Sample(np.ndarray):
+    """The recorded part of a reference output: `part` indexes it out of an array of `full_shape` whose bytes hash to
+    `digest` (sha1)."""
+
+
+def _part(shape):
+    """The fixed, seeded part of an array of `shape` that a recording keeps: an 8 x 32 window of an image, 128 columns of a
+    few-row array (the surfel rows: the first and last 16 and 96 between), 192 entries of a vector (32, 128, 32)."""
+    if len(shape) >= 2 and shape[0] > 16:
+        h, w = shape[:2]
+        return np.arange(h // 3, min(h, h // 3 + 8))[:, None], np.arange(w // 3, min(w, w // 3 + 32))[None, :]
+    n, edge, mid = shape[-1], (32, 16)[len(shape) > 1], (128, 96)[len(shape) > 1]
+    pick = np.random.default_rng(0).choice(np.arange(edge, n - edge), min(n - 2 * edge, mid), replace=False)
+    return (slice(None),) * (len(shape) - 1) + (np.concatenate([np.arange(edge), np.sort(pick), np.arange(n - edge, n)]),)
+
+
+def same_sample(a, b):
+    """(a, b) restricted to what the reference output `b` holds of the whole: unchanged unless `b` is a recorded Sample."""
+    if not isinstance(b, Sample):
+        return a, b
+    a = np.asarray(a)
+    assert a.shape == b.full_shape, (a.shape, b.full_shape)
+    assert b.part is not None, "this reference output is recorded as its digest only (DIGEST_ONLY)"
+    return a[b.part], b.view(np.ndarray)
+
+
+def identical(a, b):
+    """Bitwise equality of `a` and the reference output `b` (over the whole array through the digest of a recorded Sample)."""
+    a = np.ascontiguousarray(a)
+    if not isinstance(b, Sample):
+        b = np.ascontiguousarray(b)
+        return a.shape == b.shape and a.itemsize == b.itemsize and a.tobytes() == b.tobytes()
+    return a.shape == b.full_shape and a.itemsize == b.itemsize and hashlib.sha1(a.tobytes()).hexdigest() == b.digest
+
+
+def shape_of(b):
+    return b.full_shape if isinstance(b, Sample) else np.shape(b)
+
+
+def _test_id():
+    t = os.environ.get("PYTEST_CURRENT_TEST", "no_test").rsplit(" (", 1)[0]
+    return re.sub(r"[^A-Za-z0-9_.-]+", "_", t.split("/")[-1].replace(".py::", "__"))
+
+
+def _pack(a):
+    a = np.ascontiguousarray(a)
+    return [a.dtype.str, list(a.shape), base64.b64encode(a.tobytes()).decode()]
+
+
+def _unpack(p):
+    return np.frombuffer(base64.b64decode(p[2]), np.dtype(p[0])).reshape(p[1]).copy()
+
+
+def _encode(v, digest_only=False):
+    if v is None:
+        return ["n"]
+    if isinstance(v, (bool, np.bool_)):
+        return ["b", bool(v)]
+    if isinstance(v, (int, np.integer)):
+        return ["i", int(v)]
+    if isinstance(v, (float, np.floating)):
+        return ["f", float(v)]
+    if isinstance(v, tuple):
+        return ["t", [_encode(x) for x in v]]
+    if isinstance(v, C.Structure):
+        fields = {f: getattr(v, f) for f, _ in v._fields_}
+        return ["s", {f: _encode(np.array(x) if isinstance(x, C.Array) else x) for f, x in fields.items()}]
+    v = np.ascontiguousarray(v)
+    if v.size <= WHOLE:
+        return ["a", _pack(v)]
+    if digest_only:
+        return ["d", v.dtype.str, list(v.shape), hashlib.sha1(v.tobytes()).hexdigest()]
+    part = _part(v.shape)
+    return ["p", _pack(v[part]), list(v.shape), hashlib.sha1(v.tobytes()).hexdigest(),
+            [None if isinstance(i, slice) else _pack(i) for i in part]]
+
+
+def _decode(spec):
+    kind = spec[0]
+    if kind == "n":
+        return None
+    if kind in ("b", "i", "f"):
+        return spec[1]
+    if kind == "t":
+        return tuple(_decode(s) for s in spec[1])
+    if kind == "s":
+        import types
+        return types.SimpleNamespace(**{k: _decode(s) for k, s in spec[1].items()})
+    if kind == "a":
+        return _unpack(spec[1])
+    if kind == "d":
+        out = np.zeros(0, np.dtype(spec[1])).view(Sample)
+        out.full_shape, out.digest, out.part = tuple(spec[2]), spec[3], None
+        return out
+    out = _unpack(spec[1]).view(Sample)
+    out.full_shape, out.digest = tuple(spec[2]), spec[3]
+    out.part = tuple(slice(None) if i is None else _unpack(i) for i in spec[4])
+    return out
+
+
+class _Recording:
+    """One test's calls: per RefDirectBA (in construction order), [method, encoded result] per call, as JSON."""
+    current = None
+
+    def __init__(self, test_id, directory, replay):
+        self.test_id, self.path = test_id, os.path.join(directory, test_id + ".npz")
+        self.calls, self.used = [], []
+        if replay:
+            if not os.path.exists(self.path):
+                raise FileNotFoundError(f"no recorded reference run {self.path}: run the test once against the reference's kernels "
+                                        "(oracle/build_ref.sh) with BADBA_RECORD_REFERENCE=<dir> and store <dir>/*.npz there")
+            with np.load(self.path) as f:
+                self.calls = json.loads(f["calls"].tobytes())
+
+    @classmethod
+    def get(cls, directory, replay):
+        if cls.current is None or cls.current.test_id != _test_id():
+            cls.current = cls(_test_id(), directory, replay)
+        return cls.current
+
+    def save(self):
+        np.savez_compressed(self.path, calls=np.frombuffer(json.dumps(self.calls).encode(), np.uint8))
+
+
+class _Recorder:
+    def __init__(self, live, rec):
+        self._live, self._rec, self._i = live, rec, len(rec.calls)
+        rec.calls.append([])
+
+    def __getattr__(self, name):
+        fn = getattr(self._live, name)
+
+        def call(*args, **kw):
+            out = fn(*args, **kw)
+            log = self._rec.calls[self._i]
+            digest = DIGEST_ONLY.get(name, ())
+            log.append([name, ["t", [_encode(x, j in digest) for j, x in enumerate(out)]] if digest else _encode(out)])
+            self._rec.save()
+            return out
+        return call
+
+
+class _Replay:
+    def __init__(self, rec):
+        self._rec, self._i, self._n = rec, len(rec.used), 0
+        rec.used.append(None)
+        assert self._i < len(rec.calls), f"{rec.path}: the recording has {len(rec.calls)} reference instances, the test makes more"
+
+    def __getattr__(self, name):
+        def call(*args, **kw):
+            log = self._rec.calls[self._i]
+            assert self._n < len(log) and log[self._n][0] == name, \
+                f"{self._rec.path}: call {self._n} of reference instance {self._i} is {name}, recorded: {log[self._n][0] if self._n < len(log) else 'none'}"
+            out = _decode(log[self._n][1])
+            self._n += 1
+            return out
+        return call
+
+
+def reference(scene, *args, **kw):
+    """RefDirectBA(scene, ...) for a test: recorded into $BADBA_RECORD_REFERENCE when that is set (needs the library and a
+    GPU), otherwise replayed from tests/golden/reference/<test>.npz."""
+    out_dir = os.environ.get("BADBA_RECORD_REFERENCE")
+    if out_dir:
+        assert available(), f"{LIB_PATH} missing or no GPU (oracle/build_ref.sh)"
+        os.makedirs(out_dir, exist_ok=True)
+        return _Recorder(RefDirectBA(scene, *args, **kw), _Recording.get(out_dir, replay=False))
+    return _Replay(_Recording.get(RECORDED, replay=True))

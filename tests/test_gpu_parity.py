@@ -1,5 +1,6 @@
 """GPU parity tests (run with `-m gpu` on the B200 box): the sm_100a path, called through the C ABI, against
-(a) the reference's own CUDA kernels (oracle/_ref), (b) the CPU oracle and (c) the committed golden fixtures.
+(a) the reference's own CUDA kernels (recorded runs, tests/golden/reference), (b) the CPU oracle and (c) the committed
+golden fixtures.
 
 Tolerances (BASELINE.json north_star): 1e-4 relative on residual sums / normal-equation coefficients,
 1e-5 m / 1e-5 rad on poses; counts are integers and must match exactly unless noted.
@@ -29,14 +30,13 @@ def mods():
     from badslam_b200 import scene as S
     from badslam_b200.direct_ba import DirectBA
     from oracle import cpu_oracle, ref_cuda
-    assert ref_cuda.available(), "oracle/_ref/libbadslam_ref.so missing (oracle/build_ref.sh)"
     return S, DirectBA, cpu_oracle, ref_cuda
 
 
 def test_pose_coefficients_three_way(mods, small_scene):
     S, DirectBA, O, R = mods
     sc = small_scene
-    ba, ref, orc = DirectBA.from_scene(sc), R.RefDirectBA(sc), O.Oracle(sc)
+    ba, ref, orc = DirectBA.from_scene(sc), R.reference(sc), O.Oracle(sc)
     for k in range(sc.cfg.num_keyframes):
         pc = ba.AccumulatePoseEstimationCoeffs(k, sc.poses_init[k])
         H, b, cnt, cost = ref.pose_coeffs(k, sc.poses_init[k])
@@ -61,7 +61,7 @@ def test_single_residual_type(mods, tiny_scene, use_depth, use_desc):
     S, DirectBA, O, R = mods
     sc = tiny_scene
     ba = DirectBA.from_scene(sc, use_depth_residuals=use_depth, use_descriptor_residuals=use_desc)
-    ref = R.RefDirectBA(sc, use_depth, use_desc)
+    ref = R.reference(sc, use_depth, use_desc)
     for k in range(sc.cfg.num_keyframes):
         pc = ba.AccumulatePoseEstimationCoeffs(k, sc.poses_init[k])
         H, b, cnt, cost = ref.pose_coeffs(k, sc.poses_init[k])
@@ -70,7 +70,7 @@ def test_single_residual_type(mods, tiny_scene, use_depth, use_desc):
         assert expect == cnt
     ba.UpdateSurfelActivation(); ref.update_activation()
     ba.OptimizeGeometryIteration(); ref.optimize_geometry_iteration()
-    a, b_ = ba.GetSurfelsHost(), ref.surfels()
+    a, b_ = R.same_sample(ba.GetSurfelsHost(), ref.surfels())
     d = np.max(np.abs(a[:3] - b_[:3]), axis=0)
     if use_depth:
         assert d.max() < 2e-6
@@ -86,7 +86,7 @@ def test_single_residual_type(mods, tiny_scene, use_depth, use_desc):
 def test_estimate_frame_pose(mods, small_scene):
     S, DirectBA, O, R = mods
     sc = small_scene
-    ba, ref, orc = DirectBA.from_scene(sc), R.RefDirectBA(sc), O.Oracle(sc)
+    ba, ref, orc = DirectBA.from_scene(sc), R.reference(sc), O.Oracle(sc)
     for k in range(sc.cfg.num_keyframes):
         pp, ip, cp = ba.EstimateFramePose(None, sc.poses_init[k], k)
         pr, ir, cr = ref.estimate_frame_pose(k, sc.poses_init[k])
@@ -103,7 +103,7 @@ def test_estimate_frame_pose(mods, small_scene):
 def test_activation_and_geometry(mods, small_scene):
     S, DirectBA, O, R = mods
     sc = small_scene
-    ba, ref, orc = DirectBA.from_scene(sc), R.RefDirectBA(sc), O.Oracle(sc)
+    ba, ref, orc = DirectBA.from_scene(sc), R.reference(sc), O.Oracle(sc)
     # make keyframe 1 inactive and 2 covisible-active to exercise the activation rules
     for obj_set in (lambda k, a: ba.keyframes()[k].SetActivation(a), ref.set_activation):
         obj_set(1, 2)
@@ -111,16 +111,17 @@ def test_activation_and_geometry(mods, small_scene):
     orc.activation[1], orc.activation[2] = 2, 1
     ba.UpdateSurfelActivation(); ref.update_activation(); orc.update_activation()
     fa, fr, fo = ba.GetActiveHost(), ref.active(), orc.active[:sc.num_surfels]
-    assert np.array_equal(fa, fr) and np.array_equal(fo, fr)
-    assert 0 < fr.sum() <= sc.num_surfels
+    assert R.identical(fa, fr) and R.identical(fo, fr)
+    assert 0 < fa.sum() <= sc.num_surfels
     ba.OptimizeGeometryIteration(); ref.optimize_geometry_iteration(); orc.optimize_geometry_iteration()
     a, b_, c = ba.GetSurfelsHost(), ref.surfels(), orc.surfels[:8, :sc.num_surfels]
+    assert np.array_equal(a[4:6].view(np.uint32), sc.surfels[4:6, :sc.num_surfels].view(np.uint32))   # radius / colour untouched
+    (a, b_), (c, _), (s0, _) = (R.same_sample(x, b_) for x in (a, c, sc.surfels[:8, :sc.num_surfels]))
     assert np.max(np.abs(a[:3] - b_[:3])) < 2e-6                      # positions (m)
     assert (a[3].view(np.uint32) != b_[3].view(np.uint32)).sum() == 0  # packed normals
     assert np.max(np.abs(a[6:8] - b_[6:8])) < 2e-3                    # descriptors (range +-180)
-    assert np.array_equal(a[4:6].view(np.uint32), sc.surfels[4:6, :sc.num_surfels].view(np.uint32))   # radius / colour untouched
     assert np.max(np.abs(c[:3] - b_[:3])) < 5e-4 and (c[3].view(np.uint32) != b_[3].view(np.uint32)).mean() < 1e-3
-    moved = np.abs(b_[:3] - sc.surfels[:3, :sc.num_surfels]).max()
+    moved = np.abs(b_[:3] - s0[:3]).max()
     assert moved > 1e-4      # the step did something
 
 
@@ -128,7 +129,7 @@ def test_bundle_adjustment_against_reference(mods, small_scene):
     S, DirectBA, O, R = mods
     sc = small_scene
     K = sc.cfg.num_keyframes
-    ba, ref, ref2 = DirectBA.from_scene(sc), R.RefDirectBA(sc), R.RefDirectBA(sc)
+    ba, ref, ref2 = DirectBA.from_scene(sc), R.reference(sc), R.reference(sc)
     ro = ba.BundleAdjustment(None, False, False, False, True, True, 3, 3)
     rr = ref.bundle_adjust(True, True, 3, 3)
     rr2 = ref2.bundle_adjust(True, True, 3, 3)
@@ -150,7 +151,7 @@ def test_bundle_adjustment_against_reference(mods, small_scene):
         dt, dr = S.pose_error(ba.keyframes()[k].global_T_frame(), ref.pose(k))
         assert dt < POSE_T + 2 * self_noise and dr < POSE_R + 2 * self_noise, (k, dt, dr, self_noise)
     assert np.array_equal(ba.GetKeyframeStates()[1], ref.activation())
-    a, b_ = ba.GetSurfelsHost(), ref.surfels()
+    a, b_ = R.same_sample(ba.GetSurfelsHost(), ref.surfels())
     assert np.mean(np.abs(a[:3] - b_[:3])) < 1e-6
 
 
@@ -158,14 +159,14 @@ def test_windowed_bundle_adjustment(mods, small_scene):
     """active_keyframe_window != all keyframes: fixed activation + all surfels active (direct_ba_alternating.cc:354-372,444-446)."""
     S, DirectBA, O, R = mods
     sc = small_scene
-    ba, ref = DirectBA.from_scene(sc), R.RefDirectBA(sc)
+    ba, ref = DirectBA.from_scene(sc), R.reference(sc)
     ro = ba.BundleAdjustment(None, False, False, False, True, True, 2, 2, active_keyframe_window_start=1, active_keyframe_window_end=3)
     rr = ref.bundle_adjust(True, True, 2, 2, window_start=1, window_end=3)
     # (a keyframe whose last update sits at the 1e-6 convergence threshold may take one Gauss-Newton iteration more or less: the
     #  reference's float atomics make its own count vary from run to run, see test_bundle_adjustment_against_reference)
     assert abs(ro.pose_iterations_total - rr.pose_iterations_total) <= 2
     assert ba.GetActiveHost().all() and ref.active().all()
-    ref2 = R.RefDirectBA(sc)
+    ref2 = R.reference(sc)
     ref2.bundle_adjust(True, True, 2, 2, window_start=1, window_end=3)
     self_noise = max(max(S.pose_error(ref.pose(k), ref2.pose(k))) for k in range(sc.cfg.num_keyframes))
     for k in range(sc.cfg.num_keyframes):
@@ -299,7 +300,7 @@ def test_intrinsics_step_three_way(mods, opt_depth, opt_color):
     """OptimizeIntrinsicsCUDA (kernel_opt_intrinsics.cc:39-281): one step, ours vs the reference kernels vs the oracle."""
     S, DirectBA, O, R = mods
     sc = _distorted_scene(S, "small")
-    ba, ref, ref2, orc = DirectBA.from_scene(sc), R.RefDirectBA(sc), R.RefDirectBA(sc), O.Oracle(sc)
+    ba, ref, ref2, orc = DirectBA.from_scene(sc), R.reference(sc), R.reference(sc), O.Oracle(sc)
     # a non-zero deformation model, so that the d/da and d/dcfactor terms (kernel_opt_intrinsics.cu:97-113) are exercised
     a_init = 0.02
     cf_init = (np.random.default_rng(5).standard_normal(sc.cfactor.shape) * 0.003).astype(np.float32)
@@ -325,10 +326,11 @@ def test_intrinsics_step_three_way(mods, opt_depth, opt_color):
     assert abs(a0 - a1) < 1e-5 + 5 * a_noise, (a0, a1, a_noise)
     assert np.all(np.abs(d0 - d2) < tol_d) and np.all(np.abs(c0 - c2) < REL * np.abs(c2) + 1e-3) and abs(a0 - a2) < 1e-4
     cf0, cf1 = ba.cfactor_buffer(), ref.cfactor()
+    cs0, cf1 = R.same_sample(cf0, cf1)
     if opt_depth:
         assert np.any(d0 != np.asarray(sc.depth_K, np.float32)) and np.any(cf0 != cf_init) and abs(a0 - a_init) > 1e-3
-        assert (cf0 != 0).sum() == (cf1 != 0).sum()
-        assert np.abs(cf0 - cf1).max() < 1e-4 and np.abs(cf0 - orc.cfactor).max() < 1e-3
+        assert (cs0 != 0).sum() == (cf1 != 0).sum()
+        assert np.abs(cs0 - cf1).max() < 1e-4 and np.abs(cf0 - orc.cfactor).max() < 1e-3
     else:
         assert np.array_equal(d0, np.asarray(sc.depth_K, np.float32)) and np.array_equal(cf0, cf_init) and a0 == np.float32(a_init)
     if not opt_color:
@@ -340,7 +342,7 @@ def test_bundle_adjustment_with_intrinsics(mods):
     S, DirectBA, O, R = mods
     sc = _distorted_scene(S, "small")
     K = sc.cfg.num_keyframes
-    ba, ref, ref2 = DirectBA.from_scene(sc), R.RefDirectBA(sc), R.RefDirectBA(sc)
+    ba, ref, ref2 = DirectBA.from_scene(sc), R.reference(sc), R.reference(sc)
     ro = ba.BundleAdjustment(None, True, True, False, True, True, 3, 3)
     rr = ref.bundle_adjust(True, True, 3, 3, optimize_depth_intrinsics=True, optimize_color_intrinsics=True)
     ref2.bundle_adjust(True, True, 3, 3, optimize_depth_intrinsics=True, optimize_color_intrinsics=True)
@@ -379,7 +381,7 @@ def test_pcg_building_blocks_three_way(mods, name, distort, intr, use_desc, a_in
     sc = S.make_scene(cfg)
     K, n = cfg.num_keyframes, sc.num_surfels
     ba = DirectBA.from_scene(sc, use_descriptor_residuals=use_desc)
-    ref, orc = R.RefDirectBA(sc, True, use_desc), O.Oracle(sc, True, use_desc)
+    ref, orc = R.reference(sc, True, use_desc), O.Oracle(sc, True, use_desc)
     if a_init:
         cf = (np.random.default_rng(5).standard_normal(sc.cfactor.shape) * 0.003).astype(np.float32)
         ba.SetA(a_init); ba.SetCFactorBuffer(cf)
@@ -387,14 +389,18 @@ def test_pcg_building_blocks_three_way(mods, name, distort, intr, use_desc, a_in
         orc.model.a = a_init; orc.cfactor[:] = cf
     kw = dict(optimize_depth_intrinsics=intr, optimize_color_intrinsics=intr, gauge_keyframe=1)
     ours, theirs, cpu = ba.PCGDebug(**kw), ref.pcg_debug(**kw), orc.pcg_debug(**kw)
-    assert len(ours[0]) == len(theirs[0]) == len(cpu[0]) == 6 * (K - 1) + (3 if use_desc else 1) * n + ((5 + sc.cfactor.size + 4) if intr else 0)
+    size = len(ours[0])
+    assert size == R.shape_of(theirs[0])[0] == len(cpu[0]) == 6 * (K - 1) + (3 if use_desc else 1) * n + ((5 + sc.cfactor.size + 4) if intr else 0)
     for idx, what in enumerate(("r", "M", "p", "g")):
-        for seg, (lo, hi) in _segments(K, n, 3 if use_desc else 1, len(ours[0])).items():
-            scale = np.abs(theirs[idx][lo:hi]).max()
-            d = np.abs(ours[idx][lo:hi].astype(np.float64) - theirs[idx][lo:hi]).max() / scale
+        at, t = R.same_sample(np.arange(size), theirs[idx])     # (the entries the reference's vector was recorded at)
+        for seg, (lo, hi) in _segments(K, n, 3 if use_desc else 1, size).items():
+            sel = at[(at >= lo) & (at < hi)]
+            ts = t[(at >= lo) & (at < hi)]
+            scale = np.abs(ts).max()
+            d = np.abs(ours[idx][sel].astype(np.float64) - ts).max() / scale
             assert d < 5e-5, (what, seg, d)      # vs the reference's kernels: fp32 summation order only
             if seg != "surfel":                  # oracle (software texture filter, threshold flips): aggregated entries only
-                dc = np.abs(cpu[idx][lo:hi].astype(np.float64) - theirs[idx][lo:hi]).max() / scale
+                dc = np.abs(cpu[idx][sel].astype(np.float64) - ts).max() / scale
                 assert dc < 1e-3, (what, seg, dc)
     assert np.all(np.abs(ours[4] - theirs[4]) < 1e-5 * np.abs(theirs[4]))
     assert np.all(np.abs(cpu[4] - theirs[4]) < 1e-4 * np.abs(theirs[4]))
@@ -408,7 +414,7 @@ def test_pcg_bundle_adjustment_against_reference(mods, small_scene):
     sc = small_scene
     K = sc.cfg.num_keyframes
     # (1) 4 inner steps per outer iteration
-    ba, ref, ref2 = DirectBA.from_scene(sc), R.RefDirectBA(sc), R.RefDirectBA(sc)
+    ba, ref, ref2 = DirectBA.from_scene(sc), R.reference(sc), R.reference(sc)
     ro = ba.BundleAdjustment(None, False, False, False, True, True, 2, 2, use_pcg=True, pcg_max_inner_iterations=4, pcg_gauge_keyframe=2)
     rr = ref.bundle_adjust_pcg(min_iterations=2, max_iterations=2, max_inner_iterations=4, gauge_keyframe=2)
     ref2.bundle_adjust_pcg(min_iterations=2, max_iterations=2, max_inner_iterations=4, gauge_keyframe=2)
@@ -420,11 +426,11 @@ def test_pcg_bundle_adjustment_against_reference(mods, small_scene):
     for k in range(K):
         dt, dr = S.pose_error(pa[k], ref.pose(k))
         assert dt < 1e-5 + 3 * noise and dr < 1e-5 + 3 * noise, (k, dt, dr, noise)
-    a, b_ = ba.GetSurfelsHost(), ref.surfels()
+    a, b_ = R.same_sample(ba.GetSurfelsHost(), ref.surfels())
     assert np.abs(a[:3] - b_[:3]).max() < 1e-4 and np.abs(a[:3] - b_[:3]).mean() < 1e-6      # 8 fp32 CG steps
     assert (a[3].view(np.uint32) != b_[3].view(np.uint32)).mean() < 1e-4   # second normals update sees 1e-6-different positions
     # (2) full solves: same quality as the reference
-    ba, ref = DirectBA.from_scene(sc), R.RefDirectBA(sc)
+    ba, ref = DirectBA.from_scene(sc), R.reference(sc)
     ro = ba.BundleAdjustment(None, False, False, False, True, True, 3, 3, use_pcg=True, pcg_gauge_keyframe=0)
     rr = ref.bundle_adjust_pcg(min_iterations=3, max_iterations=3, gauge_keyframe=0)
     def rel_err(poses):
