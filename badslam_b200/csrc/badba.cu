@@ -26,10 +26,6 @@
 #include "odometry.cuh"
 #include "preprocess_tile.cuh"
 
-#ifndef BBA_POSE_PRECOMPUTE
-#define BBA_POSE_PRECOMPUTE 1   // per-surfel frames (normal, tangent points) computed once per pose step (kernels.cuh LaunchSurfelFrames)
-#endif
-
 namespace {
 
 using bba::KfDevice;
@@ -497,8 +493,7 @@ bba_status RunPoseStep(bba_handle h, const std::vector<int>& ids, const std::vec
   // The surfels do not move during a pose step: what the descriptor residual needs of a surfel alone (unpacked normal, the two
   // tangent points) is computed once here instead of once per (surfel, keyframe, Gauss-Newton iteration) pair.  Not worth a
   // launch + 9 rows of traffic for a handful of keyframes (frame tracking): the kernel then derives them per pair.
-  static const bool precompute = BBA_POSE_PRECOMPUTE && !std::getenv("BADBA_POSE_NO_PRECOMPUTE");   // (development switch for A/B runs)
-  if (precompute && h->cfg.use_descriptor_residuals && n_local >= 4 && h->surfels_size > 0) {
+  if (h->cfg.use_descriptor_residuals && n_local >= 4 && h->surfels_size > 0) {
     const uint32_t pitch = static_cast<uint32_t>(h->surfel_pitch_bytes / sizeof(float));
     if (!h->d_frames || h->frames_pitch < pitch) {
       cudaFree(h->d_frames);
@@ -721,11 +716,6 @@ bba_status BuildGeometryArgs(bba_handle h, bba::GeometryArgs* g, cudaStream_t s)
   g->kf_count = cnt;
   g->queue = h->d_geo_queue;
   g->tile_shift = 8;
-  // Keyframes per work item.  A group's images (1.5 MB per keyframe at 640x480) are what all resident warps gather from at one
-  // time; between groups a surfel's partial sums are parked in the scratch rows.  16 keeps a group's images in a fifth of the L2
-  // when millions of surfels stream past them; (development switch BADBA_GEO_GROUP for A/B runs)
-  static const int group_override = std::getenv("BADBA_GEO_GROUP") ? std::atoi(std::getenv("BADBA_GEO_GROUP")) : 0;
-  g->group = group_override;
   g->peers = (h->cfg.world_size > 1 && h->peers.count == h->cfg.world_size - 1) ? h->peers : bba::PeerSet{};
   if (!h->d_tile_epoch || h->tile_epoch_capacity < (h->surfels_size + 31u) / 32u) {
     cudaFree(h->d_tile_epoch);

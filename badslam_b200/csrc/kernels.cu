@@ -96,50 +96,15 @@ __device__ __forceinline__ cudaTextureObject_t UniformTexture(cudaTextureObject_
   return (static_cast<unsigned long long>(hi) << 32) | lo;
 }
 
-__device__ __forceinline__ void LoadKf(const KfDevice* __restrict__ kfs, int kf, KfRegs* r) {
-  const float4* p = reinterpret_cast<const float4*>(kfs + kf);
-  const float4 a = __ldg(p), b = __ldg(p + 1), c = __ldg(p + 2);
-  r->T[0] = a.x; r->T[1] = a.y; r->T[2] = a.z; r->T[3] = a.w;
-  r->T[4] = b.x; r->T[5] = b.y; r->T[6] = b.z; r->T[7] = b.w;
-  r->T[8] = c.x; r->T[9] = c.y; r->T[10] = c.z; r->T[11] = c.w;
-  const ulonglong2 q = __ldg(reinterpret_cast<const ulonglong2*>(p + 3));
-  r->depth = reinterpret_cast<const uint16_t*>(q.x);
-  r->normals = reinterpret_cast<const uint16_t*>(q.y);
-  const ulonglong2 q2 = __ldg(reinterpret_cast<const ulonglong2*>(p + 4));
-  r->tex = static_cast<cudaTextureObject_t>(q2.x);
-  r->depth_pitch = static_cast<uint32_t>(q2.y & 0xffffffffu);
-  r->normals_pitch = static_cast<uint32_t>(q2.y >> 32);
-  r->activation = __ldg(reinterpret_cast<const int*>(p + 5));
-}
-
-#ifndef BBA_POSE_FFMA2
-#define BBA_POSE_FFMA2 1   // packed fp32x2 arithmetic (sm_100 FFMA2 / FMUL2) for the rank-1 updates of H and b
-#endif
-
-#if !BBA_POSE_FFMA2
-// H += w J^T J (upper triangle, row-major), b += w r J   (gauss_newton.cuh:59-92, per thread)
-__device__ __forceinline__ void AccumulateHb(float (&acc)[kPoseAccSize], const float (&J)[6], float raw, float w) {
-  int idx = 0;
-#pragma unroll
-  for (int r = 0; r < 6; ++r) {
-    const float wj = w * J[r];
-#pragma unroll
-    for (int c = r; c < 6; ++c) acc[idx++] += wj * J[c];
-  }
-  const float wr = w * raw;
-#pragma unroll
-  for (int i = 0; i < 6; ++i) acc[21 + i] += wr * J[i];
-}
-__device__ __forceinline__ int AccSlot(int lane) { return lane; }
-#else
-// The same update with packed fp32x2 instructions (fma.rn.f32x2 / mul.rn.f32x2 -> SASS FFMA2 / FMUL2): each instruction
-// updates two adjacent coefficients.  The per-lane accumulators are kept in a PAIR-ALIGNED order --
+// H += w J^T J (upper triangle), b += w r J (gauss_newton.cuh:59-92, per thread), with packed fp32x2 instructions
+// (fma.rn.f32x2 / mul.rn.f32x2 -> SASS FFMA2 / FMUL2): each instruction updates two adjacent coefficients.  The per-lane
+// accumulators are kept in a PAIR-ALIGNED order --
 //   0..5  H00 H01 H02 H03 H04 H05 | 6..9 H12 H13 H14 H15 | 10..13 H22 H23 H24 H25 | 14,15 H34 H35 | 16,17 H44 H45 |
 //   18..23 b0..b5 | 24 H11  25 H33  26 H55 | 27..31 statistics
 // -- so that every row of the upper triangle is a run of (even, odd) column pairs of J plus at most one leading diagonal
 // element; AccSlot() maps the order back to the row-major upper triangle + b the solver reads (gauss_newton.cuh:59-92).
-// 12 FFMA2 + 3 FMUL2 + 3 FFMA + 1 FMUL per residual instead of 27 FFMA + 7 FMUL; each product / sum is rounded exactly as in the
-// scalar form.
+// 12 FFMA2 + 3 FMUL2 + 3 FFMA + 1 FMUL per residual instead of 27 FFMA + 7 FMUL; each product / sum is rounded exactly as by the
+// scalar instructions.
 typedef unsigned long long F32x2;
 __device__ __forceinline__ F32x2 Pack2(float lo, float hi) {
   F32x2 r;
@@ -156,10 +121,6 @@ __device__ __forceinline__ void Fma2(float* lo, float* hi, F32x2 a, F32x2 b) {  
   F32x2 c = Pack2(*lo, *hi);
   asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(c) : "l"(a), "l"(b));
   Unpack2(c, lo, hi);
-}
-__device__ __forceinline__ void AccumulateHbPacked(float (&acc)[kPoseAccSize], F32x2 J01, F32x2 J23, F32x2 J45, float raw, float w);
-__device__ __forceinline__ void AccumulateHb(float (&acc)[kPoseAccSize], const float (&J)[6], float raw, float w) {
-  AccumulateHbPacked(acc, Pack2(J[0], J[1]), Pack2(J[2], J[3]), Pack2(J[4], J[5]), raw, w);
 }
 __device__ __forceinline__ void AccumulateHbPacked(float (&acc)[kPoseAccSize], F32x2 J01, F32x2 J23, F32x2 J45, float raw, float w) {
   float J[6];
@@ -191,6 +152,11 @@ __device__ __forceinline__ void AccumulateHbPacked(float (&acc)[kPoseAccSize], F
   Fma2(&acc[20], &acc[21], dr, J23);
   Fma2(&acc[22], &acc[23], dr, J45);
 }
+// J reaches the update through the packed registers; taking the diagonal terms from the array instead gives the same sums but a
+// different instruction schedule of the pose kernel.
+__device__ __forceinline__ void AccumulateHb(float (&acc)[kPoseAccSize], const float (&J)[6], float raw, float w) {
+  AccumulateHbPacked(acc, Pack2(J[0], J[1]), Pack2(J[2], J[3]), Pack2(J[4], J[5]), raw, w);
+}
 // accumulator index in the pair-aligned order -> index in the solver's order (21 upper-triangle coefficients row-major, 6 b, 5 stats)
 __device__ __forceinline__ int AccSlot(int lane) {
   //            H00 H01 H02 H03 H04 H05 H12 H13 H14 H15 H22 H23 H24 H25 H34 H35 H44 H45 b0  b1  b2  b3  b4  b5 H11 H33 H55
@@ -204,45 +170,11 @@ __device__ __forceinline__ int AccSlot(int lane) {
   if (lane < 27) return static_cast<int>((hi >> (5 * (lane - 24))) & 31u);
   return lane;
 }
-#endif
 
-#ifndef BBA_POSE_UNROLL
-#define BBA_POSE_UNROLL 1
-#endif
-#ifndef BBA_POSE_MIN_CTAS
-#define BBA_POSE_MIN_CTAS 2   // resident CTAs per SM the register allocation is tuned for
-#endif
-// 2-wide (fp32x2) post-association maths (device_math.cuh: tangent points, sample coordinates, Jacobians).  OFF: measured on
-// B200 it does not shorten the kernel (3.7145 vs 3.7148 ms per launch: the kernel is bound by dependent-issue latency at 4 warps
-// per scheduler, not by the instruction count), and it rounds the texture sample coordinates differently from the reference's
-// compiled expressions -- the texture unit quantises the filter fraction to 1/256 pixel, so a last-bit change of a coordinate
-// flips the filter weights of ~1 % of the samples (residual changes of up to ~0.5 of +-180).  In the geometry kernel that cost
-// the bit-exact agreement of the surfel positions with the reference (errors up to 9e-5 m on 0.07 % of the surfels).
-#ifndef BBA_POSE_PACKED
-#define BBA_POSE_PACKED 0
-#endif
-#ifndef BBA_GEO_PACKED
-#define BBA_GEO_PACKED 0
-#endif
-#ifndef BBA_POSE_CHUNK_SHIFT
-#define BBA_POSE_CHUNK_SHIFT 8
-#endif
-constexpr int kPoseChunkShift = BBA_POSE_CHUNK_SHIFT;   // log2 of the surfels one warp evaluates per (keyframe) sub-item
-// Sub-item size chosen per ITEM from the number of keyframes in its group (so that the last, short group of a work list and the
-// tail of a Gauss-Newton loop still offer every warp a sub-item) instead of per launch.  OFF: measured on B200 at cfg3 it is
-// 0.5 % slower (pose stage 20.26 vs 20.15 ms; the extra warp reductions of the smaller chunks cost more than the idle warps of
-// the few short groups), tools/r2_gpu14.sh.
-#ifndef BBA_POSE_ITEM_CHUNKS
-#define BBA_POSE_ITEM_CHUNKS 0
-#endif
-#ifndef BBA_POSE_NOBARRIER
-#define BBA_POSE_NOBARRIER 1   // item loop without a CTA-wide barrier (the last warp out of a stage re-arms it)
-#endif
-#ifndef BBA_POSE_THREADS
-#define BBA_POSE_THREADS 256
-#endif
-constexpr int kPoseThreads = BBA_POSE_THREADS;
-constexpr int kPoseUnroll = BBA_POSE_UNROLL;   // surfels of a chunk evaluated concurrently per lane
+constexpr int kPoseThreads = 256;
+constexpr int kPoseMinCtas = 2;      // resident CTAs per SM the register allocation is tuned for
+constexpr int kPoseUnroll = 1;       // surfels of a chunk evaluated concurrently per lane
+constexpr int kPoseChunkShift = 8;   // log2 of the surfels one warp evaluates per (keyframe) sub-item
 constexpr int kPoseStagedRows = 7;   // x y z normal radius^2 d1 d2
 constexpr int kPoseStagedRowsPre = 14;   // x y z d1 d2 + the 9 frame rows (normal, tangent point 1, tangent point 2)
 constexpr int kPoseGroup = 8;        // keyframes per work item
@@ -256,7 +188,7 @@ constexpr int kPoseGroup = 8;        // keyframes per work item
 // residual count / cost only in debug mode, kernel_opt_pose.cu:312-320,373-381).
 // PRE: the per-surfel frames (unpacked normal, tangent points) are staged instead of the packed normal and the radius.
 template <int TILE, bool STATS, bool PRE>
-__global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulateKernel(const __grid_constant__ PoseAccumulateArgs args) {
+__global__ void __launch_bounds__(kPoseThreads, kPoseMinCtas) PoseAccumulateKernel(const __grid_constant__ PoseAccumulateArgs args) {
   constexpr int kRows = PRE ? kPoseStagedRowsPre : kPoseStagedRows;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float* stage_base = reinterpret_cast<float*>(smem_raw);   // [2][kRows][TILE]
@@ -273,8 +205,6 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
   const uint32_t n_tiles = (args.n + TILE - 1) / TILE;
   const uint32_t n_groups = (n_work + kPoseGroup - 1) / kPoseGroup;
   const uint32_t n_items = n_groups * n_tiles;
-  // 256-surfel chunks (one warp-level reduction per 8 steps); smaller ones when the item's group holds few keyframes, so that
-  // every warp of the CTA still finds a sub-item (the tail of a Gauss-Newton loop, the last group of a short work list)
   constexpr int kTileShift = (TILE == 1024) ? 10 : (TILE == 512) ? 9 : 8;
 
   const CameraParams& cam = args.cam;
@@ -307,11 +237,11 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
     }
   };
 
-#if BBA_POSE_NOBARRIER
   // No CTA-wide barrier in the item loop: a warp that has run out of sub-items of stage s moves on to stage s ^ 1 at once.
   // The LAST warp to leave a stage (shared-memory counter) re-arms it: claims the next item, resets the sub-item counter and
   // starts the TMA copies; everybody else finds the stage ready through its mbarrier phase.  When the queue is exhausted the
-  // stage gets a sentinel item and a plain arrive, so that the waiting warps wake up and leave.
+  // stage gets a sentinel item and a plain arrive, so that the waiting warps wake up and leave.  (A __syncthreads per item
+  // instead, with thread 0 refilling the other stage, measured 2 % slower.)
   __shared__ int s_done[2];
   constexpr int kWarps = kPoseThreads / 32;
   auto arm_stage = [&](int s) {   // one thread
@@ -336,31 +266,6 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
     MbarWait(&full_bar[s], (it >> 1) & 1);
     const unsigned int item = *reinterpret_cast<volatile unsigned int*>(&s_item[s]);
     if (item >= n_items) break;
-#else
-  if (tid == 0) {
-    MbarInit(&full_bar[0], 1);
-    MbarInit(&full_bar[1], 1);
-    FenceBarrierInit();
-    s_sub[0] = 0;
-    s_sub[1] = 0;
-    const unsigned int first = atomicAdd(args.queue, 1u);
-    s_item[0] = first;
-    if (first < n_items) issue_tile(first, 0);
-  }
-  __syncthreads();
-
-  for (uint32_t it = 0;; ++it) {
-    const int s = it & 1;
-    const unsigned int item = s_item[s];
-    if (item >= n_items) break;
-    if (tid == 0) {
-      // stage s^1 was released by the __syncthreads that ended the previous iteration
-      const unsigned int next = atomicAdd(args.queue, 1u);
-      s_item[s ^ 1] = next;
-      if (next < n_items) issue_tile(next, s ^ 1);
-    }
-    MbarWait(&full_bar[s], (it >> 1) & 1);
-#endif
 
     // staged rows: x y z normal radius^2 d1 d2, or (PRE) x y z d1 d2 + 9 frame rows
     const float* sx = stage_base + (s * kRows + 0) * TILE;
@@ -376,11 +281,10 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
     const uint32_t base = tile * TILE;
     const uint32_t cnt = min(static_cast<uint32_t>(TILE), args.n - base);
     const int kfs_in_group = min(kPoseGroup, n_work - static_cast<int>(group) * kPoseGroup);
-#if BBA_POSE_ITEM_CHUNKS
-    const int wanted_shift = kfs_in_group >= 4 ? kPoseChunkShift : (kfs_in_group >= 2 ? 7 : 6);
-#else
-    const int wanted_shift = n_work >= 4 ? kPoseChunkShift : 7;   // (round-1 rule: one size per launch; kept for A/B builds)
-#endif
+    // 256-surfel chunks (one warp-level reduction per 8 steps); 128 for a work list of fewer than 4 keyframes, so that every
+    // warp of the CTA still finds a sub-item.  Choosing the size per item, from the keyframes in its group, measured 0.5 %
+    // slower at cfg3: the extra reductions of the smaller chunks cost more than the idle warps of the few short groups.
+    const int wanted_shift = n_work >= 4 ? kPoseChunkShift : 7;
     const int chunk_shift = wanted_shift < kTileShift ? wanted_shift : kTileShift;
     const uint32_t chunk_len = 1u << chunk_shift;
     const int chunks_per_tile = TILE >> chunk_shift;
@@ -399,9 +303,6 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
       const int kf = LoadKfShared(&s_kf[s][kf_local], &K);
       K.tex = UniformTexture(K.tex);
 
-#if BBA_POSE_PACKED
-      const KfPairs KP = MakeKfPairs(K.T);
-#endif
       float acc[kPoseAccSize];
 #pragma unroll
       for (int i = 0; i < kPoseAccSize; ++i) acc[i] = 0.f;
@@ -413,11 +314,7 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
         int st = 0;
         Assoc r;
         Vec3 gp, nrm;
-#if BBA_POSE_PACKED
-        DescEval2 e2;
-#else
         DescEval e;
-#endif
         bool photo = false;
         if (j < j1) {
           gp = V3(sx[j], sy[j], sz[j]);
@@ -428,15 +325,10 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
             const PixelLoads l = LoadPixel(cam, K.depth, K.depth_pitch, K.normals, K.normals_pitch, r);
             nrm = PRE ? V3(sf[j], sf[TILE + j], sf[2 * TILE + j]) : UnpackNormal(__float_as_uint(sn[j]));
             if (cam.use_desc) {
-#if BBA_POSE_PACKED
-              const F2 c_pxy = Fma(Pack(cam.d2c_fx, cam.d2c_fy), Pack(r.pxf, r.pyf), Pack(cam.d2c_cx, cam.d2c_cy));   // DepthToColor
-              float ccx, ccy;
-              Unpack(c_pxy, &ccx, &ccy);
-              photo = ccx >= 0 && ccy >= 0 && static_cast<int>(ccx) < cam.cw && static_cast<int>(ccy) < cam.ch;
-              F2 t1, t2;
-              TangentProjections2(cam, KP, K.T, gp, nrm, sr[j], &t1, &t2);
-              EvalDescriptor2(K.tex, c_pxy, t1, t2, sd1[j], sd2[j], &e2);
-#else
+              // Scalar on purpose.  A 2-wide (fp32x2) form of the post-association maths was no faster (3.7145 vs 3.7148 ms per
+              // launch: the kernel waits on dependent-issue latency, not on the FMA pipe), and it rounds the sample coordinates
+              // differently from the reference: the texture unit quantises the filter fraction to 1/256 pixel, so a last-bit
+              // change flips the filter weights of ~1 % of the samples.
               float ccx, ccy;
               photo = DepthToColor(cam, r.pxf, r.pyf, &ccx, &ccy);
               float t1x, t1y, t2x, t2y;
@@ -447,7 +339,6 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
                 TangentProjections(cam, K.T, gp, nrm, sr[j], &t1x, &t1y, &t2x, &t2y);
               }
               EvalDescriptor(K.tex, ccx, ccy, t1x, t1y, t2x, t2y, sd1[j], sd2[j], &e);
-#endif
             }
             st = Associate(cam, K.T, nrm, l, &r);
           }
@@ -467,13 +358,6 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
             Vec3 up;
             const float raw = DepthResidual(cam, r, &inv_stddev, &up);
             // kernel_opt_pose.cu:88-93
-#if BBA_POSE_PACKED
-            const F2 inv2 = Splat(inv_stddev);
-            const F2 J01 = inv2 * Pack(r.ln.x, r.ln.y);
-            const F2 J23 = inv2 * Pack(r.ln.z, -r.ln.y * up.z + r.ln.z * up.y);
-            const F2 J45 = inv2 * Pack(r.ln.x * up.z - r.ln.z * up.x, -r.ln.x * up.y + r.ln.y * up.x);
-            AccumulateHbPacked(acc, J01.v, J23.v, J45.v, raw, DepthWeight(raw));
-#else
             float J[6];
             J[0] = inv_stddev * r.ln.x;
             J[1] = inv_stddev * r.ln.y;
@@ -482,25 +366,10 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
             J[4] = inv_stddev * (r.ln.x * up.z - r.ln.z * up.x);
             J[5] = inv_stddev * (-r.ln.x * up.y + r.ln.y * up.x);
             AccumulateHb(acc, J, raw, DepthWeight(raw));
-#endif
             if (STATS) acc[29] += DepthCost(raw);
           }
           if (cam.use_desc && photo) {
             acc[28] += 1.f;
-#if BBA_POSE_PACKED
-            const DescJacShared js = MakeDescJacShared(r.lp);
-            float r1, r2;
-            Unpack(e2.r, &r1, &r2);
-            F2 J01, J23, J45;
-            DescPoseJacobian2(cam, js, e2.g1, &J01, &J23, &J45);
-            AccumulateHbPacked(acc, J01.v, J23.v, J45.v, r1, DescWeight(r1));
-            DescPoseJacobian2(cam, js, e2.g2, &J01, &J23, &J45);
-            AccumulateHbPacked(acc, J01.v, J23.v, J45.v, r2, DescWeight(r2));
-            if (STATS) {
-              acc[30] += DescCost(r1);
-              acc[31] += DescCost(r2);
-            }
-#else
             float J[6];
             DescPoseJacobian(cam, r.lp, e.gx1, e.gy1, J);
             AccumulateHb(acc, J, e.r1, DescWeight(e.r1));
@@ -510,7 +379,6 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
               acc[30] += DescCost(e.r1);
               acc[31] += DescCost(e.r2);
             }
-#endif
           }
         }
       }
@@ -528,7 +396,6 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
         if (n_depthok) atomicAdd(args.stage_counts + 2 * kf + 1, static_cast<unsigned long long>(n_depthok));
       }
     }
-#if BBA_POSE_NOBARRIER
     __syncwarp();
     if (lane == 0) {
       __threadfence_block();   // this warp's reads of stage s are complete before the stage can be handed back
@@ -537,10 +404,6 @@ __global__ void __launch_bounds__(kPoseThreads, BBA_POSE_MIN_CTAS) PoseAccumulat
         arm_stage(s);
       }
     }
-#else
-    __syncthreads();   // every warp is done with stage s (and with s_item[s]) before either is refilled
-    if (tid == 0) s_sub[s] = 0;
-#endif
   }
 }
 
@@ -566,7 +429,7 @@ static void LaunchPoseAccumulateT(const PoseAccumulateArgs& args, int sm_count, 
     cudaFuncSetAttribute(PoseAccumulateKernel<TILE, STATS, PRE>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     configured = true;
   }
-  PoseAccumulateKernel<TILE, STATS, PRE><<<BBA_POSE_MIN_CTAS * sm_count, kPoseThreads, smem, stream>>>(args);   // persistent
+  PoseAccumulateKernel<TILE, STATS, PRE><<<kPoseMinCtas * sm_count, kPoseThreads, smem, stream>>>(args);   // persistent
 }
 
 template <bool STATS>
@@ -574,7 +437,7 @@ static void LaunchPoseAccumulateS(const PoseAccumulateArgs& args, int sm_count, 
   // Tile size: as large as possible (one group of TMA transactions per item), but small enough that a keyframe group still
   // yields several items per resident CTA.  With the precomputed frames 14 rows are staged: 512 surfels x 2 stages = 56 KB per
   // CTA (two CTAs per SM), the same footprint as 1024 surfels of the 7-row variant.
-  const uint64_t slots = static_cast<uint64_t>(BBA_POSE_MIN_CTAS * sm_count) * 4;
+  const uint64_t slots = static_cast<uint64_t>(kPoseMinCtas * sm_count) * 4;
   if (args.frames != nullptr) {
     if (args.n >= slots * 512) LaunchPoseAccumulateT<512, STATS, true>(args, sm_count, stream);
     else LaunchPoseAccumulateT<256, STATS, true>(args, sm_count, stream);
@@ -621,16 +484,11 @@ void LaunchSurfelFrames(const float* surfels, uint32_t pitch, uint32_t n, float*
 // reference uses for exactly this purpose, kernels.cuh:78-86); a per-tile epoch word orders (group g, tile t) after
 // (group g-1, tile t).  With K <= 16 there is a single group and no scratch traffic at all.
 
-#ifndef BBA_GEO_GROUP
-#define BBA_GEO_GROUP 16
-#endif
-// (surfel, keyframe) pairs a thread of the activation / normals kernel keeps in flight.  Measured at cfg3: 1 -> 2.26 ms (64
-// registers, 32 warps / SM), 2 -> 2.54 ms (78 registers, 24 warps / SM); before the gathers were un-sunk and the records staged: 2.97 ms.
-#ifndef BBA_GEO_INTERLEAVE
-#define BBA_GEO_INTERLEAVE 1
-#endif
 constexpr int kGeoThreads = 256;
-constexpr int kGeoGroup = BBA_GEO_GROUP;   // keyframes per work item
+// Keyframes per work item.  A group's images (1.5 MB per keyframe at 640x480) are what all resident warps gather from at one
+// time; 16 keeps them in a fifth of the L2.  32 / 64 / 200 moved the two geometry kernels by -10 % ... +38 % on one rank's share
+// of an 8-GPU cfg3 job, none better for both.
+constexpr int kGeoGroup = 16;
 
 __device__ __forceinline__ unsigned int LoadAcquire(const unsigned int* p) {
   unsigned int v;
@@ -684,7 +542,9 @@ __device__ __forceinline__ void StoreActiveFlag(const GeometryArgs& a, uint32_t 
 
 // The <= kGeoGroup keyframe records of a work item, copied once per item into the warp's own shared-memory slice (coalesced
 // 16-byte loads; the per-keyframe reads in the pair loop are then conflict-free broadcasts with a fixed ~25-cycle latency
-// instead of a chain of dependent L1 accesses: keyframe id -> record row 2 -> rows 0, 1 -> image pointers).
+// instead of a chain of dependent L1 accesses: keyframe id -> record row 2 -> rows 0, 1 -> image pointers).  Staging all
+// records of the launch once per CTA instead measured slower (position + descriptor 4.76 vs 4.58 ms at cfg3): the per-warp
+// slices keep the records a warp reads next to each other.
 __device__ __forceinline__ void StageGroupRecords(const KfDevice* __restrict__ kfs, const int* __restrict__ kf_list, int count,
                                                   KfDevice* dst, int lane) {
   constexpr int kWords = sizeof(KfDevice) / 16;
@@ -702,31 +562,7 @@ __device__ __forceinline__ void StageGroupRecords(const KfDevice* __restrict__ k
   __syncwarp();
 }
 
-// The records of ALL keyframes of the launch, copied once per CTA (persistent grid) when they fit the shared-memory budget,
-// instead of a coalesced copy + an L2 round trip per (group, tile) item.  OFF: measured on B200 (tools/r2_gpu14.sh) it does not
-// pay -- position + descriptor 4.76 vs 4.58 ms at cfg3 and 0.81 vs 0.77 ms on one rank's share of an 8-GPU job (cfg3_rank8),
-// activation + normals unchanged: the per-warp slices keep the records a warp reads next to each other, the 19 KB block does not.
-// With it on, GeometryArgs::group (keyframes per work item, BADBA_GEO_GROUP) becomes a runtime choice: 32 / 64 / 200 instead of
-// 16 moved the two kernels by -10 % / +2 % ... +0 % / +38 % at cfg3_rank8, i.e. no setting beats 16 for both.
-#ifndef BBA_GEO_STAGE_ALL
-#define BBA_GEO_STAGE_ALL 0
-#endif
-constexpr int kGeoStageAllMax = 48 * 1024 / static_cast<int>(sizeof(KfDevice));   // 512 keyframes
-__device__ __forceinline__ void StageAllRecords(const KfDevice* __restrict__ kfs, const int* __restrict__ kf_list, int count, KfDevice* dst) {
-  constexpr int kWords = sizeof(KfDevice) / 16;
-  for (int idx = threadIdx.x; idx < count * kWords; idx += blockDim.x) {
-    const int rec = idx / kWords, part = idx - rec * kWords;
-    const int kf = __ldg(kf_list + rec);
-    reinterpret_cast<uint4*>(dst + rec)[part] = __ldg(reinterpret_cast<const uint4*>(kfs + kf) + part);
-  }
-  __syncthreads();
-}
-__host__ __device__ inline bool GeoStageAll(int kf_count) { return BBA_GEO_STAGE_ALL && kf_count <= kGeoStageAllMax; }
-// Keyframes per work item: the launcher's choice (GeometryArgs::group) when all records sit in shared memory, else the size of the
-// per-warp record slices.
-__host__ __device__ inline int GeoGroupSize(const GeometryArgs& a) { return (GeoStageAll(a.kf_count) && a.group > 0) ? a.group : kGeoGroup; }
-
-// One (surfel, keyframe) pair between "gathers issued" and "gathers consumed": two of them are kept in flight per thread.
+// One (surfel, keyframe) pair between "gathers issued" and "gathers consumed".
 struct PendingPair {
   bool in_image;
   Assoc r;
@@ -735,24 +571,21 @@ struct PendingPair {
 
 template <bool DETERMINE, bool NORMALS>
 __global__ void __launch_bounds__(kGeoThreads) ActivationNormalsKernel(const __grid_constant__ GeometryArgs a) {
-  extern __shared__ __align__(16) unsigned char geo_smem[];   // all records, or one kGeoGroup-record slice per warp
+  extern __shared__ __align__(16) unsigned char geo_smem[];   // one kGeoGroup-record slice per warp
   KfDevice* s_kfs = reinterpret_cast<KfDevice*>(geo_smem);
   const uint32_t tile_len = 1u << a.tile_shift;
   const uint32_t n_tiles = (a.end - a.begin + tile_len - 1) >> a.tile_shift;
-  const bool stage_all = GeoStageAll(a.kf_count);
-  const int G = GeoGroupSize(a);   // keyframes per work item
-  const uint32_t n_groups = (a.kf_count + G - 1) / G;
+  const uint32_t n_groups = (a.kf_count + kGeoGroup - 1) / kGeoGroup;
   const uint32_t n_items = n_groups * n_tiles;
   const size_t P = a.pitch;
   const int lane = threadIdx.x & 31;
-  if (stage_all) StageAllRecords(a.kfs, a.kf_list, a.kf_count, s_kfs);
   uint32_t group, tile;
   while (NextGeoItem(a, n_tiles, n_items, &group, &tile)) {
     const bool first = group == 0, last = group + 1 == n_groups;
-    const int j_begin = group * G, j_end = min(a.kf_count, static_cast<int>(group + 1) * G);
+    const int j_begin = group * kGeoGroup, j_end = min(a.kf_count, static_cast<int>(group + 1) * kGeoGroup);
     const int n_kf = j_end - j_begin;
-    KfDevice* recs = stage_all ? s_kfs + j_begin : s_kfs + (threadIdx.x >> 5) * kGeoGroup;
-    if (!stage_all) StageGroupRecords(a.kfs, a.kf_list + j_begin, n_kf, recs, lane);
+    KfDevice* recs = s_kfs + (threadIdx.x >> 5) * kGeoGroup;
+    StageGroupRecords(a.kfs, a.kf_list + j_begin, n_kf, recs, lane);
     for (uint32_t sub = 0; sub < tile_len / 32; ++sub) {
       const uint32_t li = a.begin + (tile << a.tile_shift) + sub * 32 + lane;
       const uint32_t i = SurfelShardToGlobal(li, a.shard_rank, a.shard_world);
@@ -773,8 +606,9 @@ __global__ void __launch_bounds__(kGeoThreads) ActivationNormalsKernel(const __g
       if (NORMALS || !act) {   // activation alone stops at the first association with an active keyframe
         const Vec3 gp = V3(a.surfels[kRowX * P + i], a.surfels[kRowY * P + i], a.surfels[kRowZ * P + i]);
         const Vec3 nrm = UnpackNormal(__float_as_uint(a.surfels[kRowNormal * P + i]));
-        // Two keyframes per step: both projections, then both pixels' gathers, then the association tests and the sums in
-        // keyframe order (the summation order -- and with it the result -- is the reference's: one thread, ascending keyframes).
+        // The sums in keyframe order: the summation order -- and with it the result -- is the reference's (one thread,
+        // ascending keyframes).  Two pairs in flight per thread measured slower at cfg3: 78 instead of 64 registers, 24
+        // instead of 32 warps / SM, 2.54 instead of 2.26 ms.
         auto issue = [&](const KfRegs& K, PendingPair* p) {
           p->in_image = (NORMALS || K.activation == 0) && ProjectIntoImage(a.cam, K.T, gp, &p->r);   // activation only looks at kActive keyframes
           if (p->in_image) p->l = LoadPixel(a.cam, K.depth, K.depth_pitch, K.normals, K.normals_pitch, p->r);
@@ -791,23 +625,6 @@ __global__ void __launch_bounds__(kGeoThreads) ActivationNormalsKernel(const __g
             s3 += 1.f;
           }
         };
-#if BBA_GEO_INTERLEAVE == 2
-        for (int j = 0; j < n_kf; j += 2) {
-          KfRegs K0, K1;
-          PendingPair p0, p1;
-          LoadKfShared(recs + j, &K0);
-          issue(K0, &p0);
-          p1.in_image = false;
-          if (j + 1 < n_kf) {
-            LoadKfShared(recs + j + 1, &K1);
-            issue(K1, &p1);
-          }
-          consume(K0, &p0);
-          if (!NORMALS && act) break;
-          consume(K1, &p1);
-          if (!NORMALS && act) break;
-        }
-#else
         for (int j = 0; j < n_kf; ++j) {
           KfRegs K0;
           PendingPair p0;
@@ -816,7 +633,6 @@ __global__ void __launch_bounds__(kGeoThreads) ActivationNormalsKernel(const __g
           consume(K0, &p0);
           if (!NORMALS && act) break;
         }
-#endif
       }
       if (!last) {
         if (NORMALS) {
@@ -842,23 +658,20 @@ __global__ void __launch_bounds__(kGeoThreads) ActivationNormalsKernel(const __g
 
 template <bool USE_DEPTH, bool USE_DESC>
 __global__ void __launch_bounds__(kGeoThreads, 3) PositionDescriptorKernel(const __grid_constant__ GeometryArgs a) {
-  extern __shared__ __align__(16) unsigned char geo_smem[];
+  extern __shared__ __align__(16) unsigned char geo_smem[];   // one kGeoGroup-record slice per warp
   KfDevice* s_kfs = reinterpret_cast<KfDevice*>(geo_smem);
-  const bool stage_all = GeoStageAll(a.kf_count);
-  if (stage_all) StageAllRecords(a.kfs, a.kf_list, a.kf_count, s_kfs);
   const uint32_t tile_len = 1u << a.tile_shift;
   const uint32_t n_tiles = (a.end - a.begin + tile_len - 1) >> a.tile_shift;
-  const int G = GeoGroupSize(a);
-  const uint32_t n_groups = (a.kf_count + G - 1) / G;
+  const uint32_t n_groups = (a.kf_count + kGeoGroup - 1) / kGeoGroup;
   const uint32_t n_items = n_groups * n_tiles;
   const size_t P = a.pitch;
   const int lane = threadIdx.x & 31;
   uint32_t group, tile;
   while (NextGeoItem(a, n_tiles, n_items, &group, &tile)) {
     const bool first = group == 0, last = group + 1 == n_groups;
-    const int j_begin = group * G, j_end = min(a.kf_count, static_cast<int>(group + 1) * G);
-    KfDevice* recs = stage_all ? s_kfs + j_begin : s_kfs + (threadIdx.x >> 5) * kGeoGroup;
-    if (!stage_all) StageGroupRecords(a.kfs, a.kf_list + j_begin, j_end - j_begin, recs, lane);
+    const int j_begin = group * kGeoGroup, j_end = min(a.kf_count, static_cast<int>(group + 1) * kGeoGroup);
+    KfDevice* recs = s_kfs + (threadIdx.x >> 5) * kGeoGroup;
+    StageGroupRecords(a.kfs, a.kf_list + j_begin, j_end - j_begin, recs, lane);
     for (uint32_t sub = 0; sub < tile_len / 32; ++sub) {
       const uint32_t li = a.begin + (tile << a.tile_shift) + sub * 32 + lane;
       const uint32_t i = SurfelShardToGlobal(li, a.shard_rank, a.shard_world);
@@ -904,25 +717,13 @@ __global__ void __launch_bounds__(kGeoThreads, 3) PositionDescriptorKernel(const
         DescEval e;
         bool photo = false;
         if (USE_DESC) {
-#if BBA_GEO_PACKED
-          const F2 c_pxy = Fma(Pack(a.cam.d2c_fx, a.cam.d2c_fy), Pack(r.pxf, r.pyf), Pack(a.cam.d2c_cx, a.cam.d2c_cy));   // DepthToColor
-          float ccx, ccy;
-          Unpack(c_pxy, &ccx, &ccy);
-          photo = ccx >= 0 && ccy >= 0 && static_cast<int>(ccx) < a.cam.cw && static_cast<int>(ccy) < a.cam.ch;
-          F2 t1, t2;
-          TangentProjections2(a.cam, MakeKfPairs(K.T), K.T, gp, nrm, radius_sq, &t1, &t2);
-          DescEval2 e2;
-          EvalDescriptor2(K.tex, c_pxy, t1, t2, d1, d2, &e2);
-          Unpack(e2.r, &e.r1, &e.r2);
-          Unpack(e2.g1, &e.gx1, &e.gy1);
-          Unpack(e2.g2, &e.gx2, &e.gy2);
-#else
+          // Scalar on purpose (see PoseAccumulateKernel): a 2-wide form of this maths lost the bit-exact agreement of the
+          // surfel positions with the reference (errors up to 9e-5 m on 0.07 % of the surfels).
           float ccx, ccy;
           photo = DepthToColor(a.cam, r.pxf, r.pyf, &ccx, &ccy);
           float t1x, t1y, t2x, t2y;
           TangentProjections(a.cam, K.T, gp, nrm, radius_sq, &t1x, &t1y, &t2x, &t2y);
           EvalDescriptor(K.tex, ccx, ccy, t1x, t1y, t2x, t2y, d1, d2, &e);
-#endif
         }
         if (Associate(a.cam, K.T, nrm, l, &r) != 3) continue;
         if (USE_DEPTH) {
@@ -1010,17 +811,15 @@ __global__ void __launch_bounds__(kGeoThreads, 3) PositionDescriptorKernel(const
   }
 }
 
+constexpr size_t kGeoSmemBytes = sizeof(KfDevice) * (kGeoThreads / 32) * kGeoGroup;   // one record slice per warp
+
 // Persistent grid: as many CTAs as can be co-resident (the epoch wait relies on every launched CTA being scheduled).
 // The tile (the unit one warp walks through, 32..256 surfels) is chosen so that every keyframe group offers several
 // items per resident warp: with too few tiles the per-tile epoch chain serialises the groups (seen at 2+ ranks).
-static size_t GeoSmemBytes(int kf_count) {
-  return sizeof(KfDevice) * (GeoStageAll(kf_count) ? static_cast<size_t>(kf_count) : static_cast<size_t>(kGeoThreads / 32) * kGeoGroup);
-}
-
 template <typename Kernel>
 static uint32_t GeoGrid(Kernel kernel, GeometryArgs* a, int sm_count) {
   int per_sm = 0;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kGeoThreads, GeoSmemBytes(a->kf_count));
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kGeoThreads, kGeoSmemBytes);
   if (per_sm < 1) per_sm = 1;
   const uint64_t resident_warps = static_cast<uint64_t>(per_sm) * sm_count * (kGeoThreads / 32);
   const uint32_t n = a->end - a->begin;
@@ -1028,8 +827,7 @@ static uint32_t GeoGrid(Kernel kernel, GeometryArgs* a, int sm_count) {
   while (shift > 5 && 2 * static_cast<uint64_t>((n + (1u << shift) - 1) >> shift) < 3 * resident_warps) --shift;
   a->tile_shift = shift;
   const uint32_t n_tiles = (n + (1u << shift) - 1) >> shift;
-  const int G = GeoGroupSize(*a);
-  const uint32_t n_groups = (a->kf_count + G - 1) / G;
+  const uint32_t n_groups = (a->kf_count + kGeoGroup - 1) / kGeoGroup;
   const uint64_t n_items = static_cast<uint64_t>(n_tiles) * (n_groups ? n_groups : 1);
   const uint64_t ctas_needed = (n_items + kGeoThreads / 32 - 1) / (kGeoThreads / 32);   // one item per warp
   return static_cast<uint32_t>(std::min<uint64_t>(ctas_needed, static_cast<uint64_t>(per_sm) * sm_count));
@@ -1045,7 +843,7 @@ template <typename Kernel>
 static void LaunchGeo(Kernel kernel, GeometryArgs a, int sm_count, cudaStream_t stream) {
   const uint32_t grid = GeoGrid(kernel, &a, sm_count);
   PrepareGeo(a, stream);
-  kernel<<<grid, kGeoThreads, GeoSmemBytes(a.kf_count), stream>>>(a);
+  kernel<<<grid, kGeoThreads, kGeoSmemBytes, stream>>>(a);
 }
 
 void LaunchActivationAndNormals(const GeometryArgs& a, int sm_count, bool determine_activation, bool update_normals, cudaStream_t stream) {

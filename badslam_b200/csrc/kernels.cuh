@@ -87,7 +87,6 @@ struct GeometryArgs {
   unsigned int* queue;         // work-item counter (reset by the launcher)
   unsigned int* tile_epoch;    // [ceil(n / 32)] keyframe groups retired per tile (reset by the launcher)
   int tile_shift;              // log2(surfels per tile), 5..8; chosen by the launcher
-  int group;                   // keyframes per work item (0: the default of 16); honoured when all records fit shared memory
   PeerSet peers;
 };
 // SetSurfelInactive + DetermineActiveSurfels (kernel_surfel_activation.cu:38-79) fused with the normal

@@ -1,6 +1,8 @@
 #!/usr/bin/env bash
-# Builds a variant of libbadba_b200.so with extra nvcc flags for kernels.cu into tools/ab/<name>.so (A/B experiments).
-#   tools/ab_build.sh ctas3 -DBBA_POSE_MIN_CTAS=3
+# Builds libbadba_b200.so of the current tree into tools/ab/<name>.so, so that an edited tree can be A/B-compared against it:
+#   python -m badslam_b200.build && tools/ab_build.sh base        # before the edit
+#   python -m badslam_b200.build && python tools/ab_fast.py tools/ab/base.so
+# kernels.cu is compiled afresh (with any extra nvcc flags given after the name); the other units are linked from badslam_b200/_obj.
 set -euo pipefail
 cd "$(dirname "${BASH_SOURCE[0]}")/.."
 name="$1"; shift

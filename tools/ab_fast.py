@@ -87,10 +87,7 @@ def main():
         os.remove(ref_poses)
     for lib in ["in-tree"] + libs:
         env = dict(os.environ)
-        if lib.startswith("env:"):          # the in-tree library with an environment switch, e.g. env:BADBA_POSE_NO_PRECOMPUTE=1
-            k, v = lib[4:].split("=", 1)
-            env[k] = v
-        elif lib != "in-tree":
+        if lib != "in-tree":
             env["BADBA_LIB"] = os.path.join(ROOT, lib)
         t0 = time.time()
         p = subprocess.run([sys.executable, os.path.abspath(__file__), "--child", scene_path, str(steps), ref_poses], env=env,
